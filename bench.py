@@ -138,6 +138,24 @@ def make_input(w, seed, ntime=None):
     return x
 
 
+def dump_output(dirname, name, a, keep):
+    """--dump-outputs: `a` as dirname/name.npy in float32, on `keep` of its
+    columns (last axis), a fixed seeded choice, so the dump stays small and
+    two runs with the same arguments write the same elements."""
+    a = np.asarray(a)
+    if keep < a.shape[-1]:
+        idx = np.sort(np.random.default_rng(0).choice(a.shape[-1], keep, replace=False))
+        a = a[..., idx]
+    os.makedirs(dirname, exist_ok=True)
+    np.save(os.path.join(dirname, name + '.npy'), np.ascontiguousarray(a, dtype=np.float32))
+
+
+# columns of the dispersion bank kept by --dump-outputs: [max_delay, 8192] f32 (26 MB at max_delay 794)
+DUMP_BANK_COLUMNS = 8192
+# of the spectrometer's [4, 4096 * 1024] f32 output: [4, 2**20] (16 MB)
+DUMP_SPECTRA_COLUMNS = 2 ** 20
+
+
 class ClockSampler(object):
     """nvidia-smi clocks/throttle reasons sampled during the timed region."""
     QUERY = ('clocks.sm,clocks.max.sm,power.draw,clocks_event_reasons.hw_slowdown,'
@@ -434,7 +452,10 @@ def oracle_window_check(x, got_fn, w, windows):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument('--gpus', type=int, default=1)
-    ap.add_argument('--steps', type=int, default=20)
+    ap.add_argument('--steps', type=int, default=20,
+                    help='timed steps of each figure: the resident FDMT step, e2e and the spectrometer chain '
+                         '(N > 1: the strong-scaling step and e2e; the per-phase, full-band and replica '
+                         'breakdowns time a fixed 5 or 10)')
     ap.add_argument('--warmup', type=int, default=3)
     ap.add_argument('--impl', default='b200', choices=['b200', 'reference'])
     ap.add_argument('--no-cpu-baseline', action='store_true')
@@ -445,8 +466,16 @@ def main():
     ap.add_argument('--no-traffic', action='store_true')
     ap.add_argument('--no-gpu-reference', action='store_true')
     ap.add_argument('--dry-run', action='store_true')
+    ap.add_argument('--dump-outputs', metavar='DIR',
+                    help='write what the last timed step computed to DIR/<name>.npy (float32): fdmt_bank = '
+                         'the dispersion bank (N > 1: the gathered one), spectrometer = the fused chain\'s '
+                         'output, each on a fixed seeded sample of its columns')
     ap.add_argument('--traffic-probe', action='store_true', help=argparse.SUPPRESS)
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
+    if args.dump_outputs and (args.impl == 'reference' or args.dry_run):
+        ap.error('--dump-outputs writes what the GPU arm computes')
     args.warmup = max(args.warmup, 3) if args.impl == 'b200' else args.warmup
 
     rank = int(os.environ.get('RANK', '0'))
@@ -558,6 +587,8 @@ def main():
     ms_step = ms_total / args.steps
     launches_per_step = max(1, launches // args.steps)
     log('resident ms/step', ms_step)
+    if args.dump_outputs:                          # before anything below reuses d_out
+        dump_output(args.dump_outputs, 'fdmt_bank', d_out.copy('system'), keep=DUMP_BANK_COLUMNS)
 
     # value check of exactly this gulp (untimed): five windows, both edges
     got_dev = d_out
@@ -567,9 +598,8 @@ def main():
     parity = oracle_window_check(x_host, got_fn, w, [(0, 4096), (40000, 4096), (65536 + 3, 4096), (100001, 4096),
                                                        (ntime - 4096 - md, 4096 + md)])
 
-    e2e_steps = max(4, min(args.steps, 10))
-    ms_e2e_total, _, _ = timed(step_e2e, 2, e2e_steps)
-    ms_e2e_serial = ms_e2e_total / e2e_steps
+    ms_e2e_total, _, _ = timed(step_e2e, 2, args.steps)
+    ms_e2e_serial = ms_e2e_total / args.steps
 
     # The same three calls as a host pipeline, the way bifrost runs blocks: one
     # thread (and thread-local stream) per stage -- copy(H2D) -> fdmt -> copy(D2H)
@@ -636,7 +666,7 @@ def main():
 
     try:
         run_pipeline(2)                                # warm-up
-        ms_pipe = run_pipeline(e2e_steps) / e2e_steps
+        ms_pipe = run_pipeline(args.steps) / args.steps
     except Exception as e:                             # keep the serial figure
         log('pipelined e2e failed:', e)
         ms_pipe = float('inf')
@@ -672,7 +702,7 @@ def main():
     chain = None
     if not args.no_chain:
         del ws
-        chain = time_chain(bf, torch, timed, peaks)
+        chain = time_chain(bf, torch, timed, peaks, args.steps, args.dump_outputs)
 
     cpu = None
     if not args.no_cpu_baseline:
@@ -740,10 +770,11 @@ def time_gpu_reference(bf, torch, stream, d_in, d_out, w):
         return dict(available=False, note=f'reference library failed: {e}')
 
 
-def time_chain(bf, torch, timed, peaks):
+def time_chain(bf, torch, timed, peaks, nstep, dump_dir=None):
     nframe, cchan, nfft, f_avg = 32, 4096, 4096, 4
     nbyte = nframe * cchan * nfft * 4
-    raw = torch.randint(-127, 128, (nbyte,), dtype=torch.int8, device='cuda')
+    gen = torch.Generator(device='cuda').manual_seed(1234)
+    raw = torch.randint(-127, 128, (nbyte,), dtype=torch.int8, device='cuda', generator=gen)
     xg = bf.empty((nframe, cchan, nfft, 2), 'ci8', 'cuda')
     from bifrost_b200.libbifrost import _bf, _check
     _check(_bf.bfMemcpy(xg.ctypes.data, xg.as_BFarray().space, raw.data_ptr(),
@@ -751,8 +782,10 @@ def time_chain(bf, torch, timed, peaks):
     torch.cuda.synchronize()
     del raw
     og = bf.zeros((4, cchan * nfft // f_avg), 'f32', 'cuda')
-    ms_c, _, _ = timed(lambda: bf.spectrometer(xg, og, nfft, f_avg, 0.0), 3, 10)
-    ms_c /= 10
+    ms_c, _, _ = timed(lambda: bf.spectrometer(xg, og, nfft, f_avg, 0.0), 3, nstep)
+    ms_c /= nstep
+    if dump_dir:
+        dump_output(dump_dir, 'spectrometer', og.copy('system'), keep=DUMP_SPECTRA_COLUMNS)
     gbs = nbyte / (ms_c * 1e-3) / 1e9
     # useful fp32 work: 2 pols x 5 N log2 N per 4096-point FFT + detect/reduce (~16 flop/sample)
     flops = nframe * cchan * (2 * 5 * nfft * 12 + 16 * nfft)
@@ -818,6 +851,8 @@ def run_multi(args, rank, local_rank, world, bf, Fdmt, torch, dist, stream, time
 
     ms_total, launches, clocks = timed(step_strong, args.warmup, args.steps, sampler, post=compute)
     ms_step = ms_total / args.steps
+    if args.dump_outputs and rank == 0:
+        dump_output(args.dump_outputs, 'fdmt_bank', t_bank.cpu().numpy(), keep=DUMP_BANK_COLUMNS)
     ms_scatter = timed(scatter, 2, 5)[0] / 5
     ms_compute = timed(compute, 2, 5)[0] / 5
     ms_gather = timed(gather, 2, 5)[0] / 5
@@ -855,8 +890,7 @@ def run_multi(args, rank, local_rank, world, bf, Fdmt, torch, dist, stream, time
         if rank == 0:
             bf.copy_array(pinned_bank, a_bank)
 
-    e2e_steps = max(4, min(args.steps, 10))
-    ms_e2e = timed(step_e2e, 2, e2e_steps)[0] / e2e_steps
+    ms_e2e = timed(step_e2e, 2, args.steps)[0] / args.steps
     del pinned_in, pinned_bank
 
     # cross-GPU FULL-BAND transform of the same gulp (SURVEY 8f.1): every rank

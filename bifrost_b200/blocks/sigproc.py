@@ -91,6 +91,10 @@ class SigprocSinkBlock(SinkBlock):
         hdr = {}
         for key in ('source_name', 'rawdatafile', 'az_start', 'za_start'):
             _copy_item_if_exists(hdr, ihdr, key)
+        if hdr.get('rawdatafile') is not None:
+            # the file's name, as for the output file below: a source block's full
+            # path can be longer than the 79 bytes a sigproc header string holds
+            hdr['rawdatafile'] = os.path.basename(str(hdr['rawdatafile']))
         _copy_item_if_exists(hdr, ihdr, 'raj', 'src_raj')
         _copy_item_if_exists(hdr, ihdr, 'dej', 'src_dej')
         if ihdr.get('telescope') is not None:

@@ -57,12 +57,17 @@ def _write_string(f, text):
 
 
 def write_header(hdr, f):
-    """Keys with value None are skipped; unknown keys warn (sigproc2.py:180-199)."""
+    """Keys with value None are skipped; unknown keys warn (sigproc2.py:180-199).
+    A string value of 80 bytes or more is an error: no sigproc reader (this
+    one, the reference's, SIGPROC's 80-character fields) can read it back."""
     _write_string(f, "HEADER_START")
     for key, val in hdr.items():
         if val is None:
             continue
         if key in _string_values:
+            if len(val.encode()) >= 80:
+                raise ValueError("sigproc header %s is %d bytes; readers take at most 79: %r"
+                                 % (key, len(val.encode()), val))
             _write_string(f, key)
             _write_string(f, val)
         elif key in _double_values:

@@ -1,12 +1,14 @@
 """Generates tests/golden/fdmt_ref_golden.npz by running the REFERENCE's own
-CUDA FDMT (oracle/_ref/libbifrost_ref.so, built from /root/reference/src by
-oracle/ref_build.sh) on seeded inputs.  Needs a GPU:
+CUDA FDMT (oracle/_ref/libbifrost_ref.so, built by oracle/ref_build.sh) on
+seeded inputs.  Needs a GPU:
 
-    gpurun -- 'python tests/golden/make_fdmt_golden.py gpurun_out/fdmt_ref_golden.npz'
+    python tests/golden/make_fdmt_golden.py OUT.npz
 
-then copy the file to tests/golden/.  The reference's tests hold no FDMT
-known-answer vector (test/test_fdmt.py:49-65 is a smoke test), so these
-outputs are what pins the oracle (oracle/fdmt.py) for this op.
+then copy OUT.npz to tests/golden/fdmt_ref_golden.npz.  The reference's tests
+hold no FDMT known-answer vector (test/test_fdmt.py:49-65 is a smoke test), so
+these outputs are what pins the oracle (oracle/fdmt.py) for this op.  Each
+output is stored as its digest and a sample (tests/golden/digest.py); the
+inputs are regenerated from their seeds by make_input().
 """
 import ctypes
 import os
@@ -50,6 +52,7 @@ def make_input(name, shape, dtype, seed):
 def main(out_path):
     import bifrost_b200 as bf
     from bifrost_b200.libbifrost import _check
+    from golden import digest
     import reflib
     ref = reflib.load()
     assert ref is not None, "oracle/_ref/libbifrost_ref.so missing: run oracle/ref_build.sh"
@@ -67,12 +70,12 @@ def main(out_path):
         bf.device.stream_synchronize()
         out = d_out.copy('system')
         _check(ref.bfFdmtDestroy(plan))
-        store[name + '/in'] = x
-        store[name + '/out'] = np.asarray(out)
+        store.update(digest.pack(name + '/out', np.asarray(out), exact=True))
         print(name, 'ok', np.asarray(out).shape)
     np.savez_compressed(out_path, **store)
     print('wrote', out_path)
 
 
 if __name__ == '__main__':
-    main(sys.argv[1] if len(sys.argv) > 1 else os.path.join(ROOT, 'gpurun_out', 'fdmt_ref_golden.npz'))
+    main(sys.argv[1] if len(sys.argv) > 1 else os.path.join(os.path.dirname(os.path.abspath(__file__)),
+                                                            'fdmt_ref_golden.npz'))

@@ -1,8 +1,8 @@
 """Generates tests/golden/io_golden.json from the REFERENCE's own Python
 (python/bifrost/sigproc2.py write_header / _read_header, guppi_raw.py
-read_header), executed from /root/reference with its `bifrost.telemetry` import
-stubbed out (the package itself cannot be imported without libbifrost).
-Run in the build container only; the tests read the committed JSON."""
+read_header), executed from the reference checkout ($BIFROST_REFERENCE, by default
+/root/reference) with its `bifrost.telemetry` import stubbed out (the package
+itself cannot be imported without libbifrost).  The tests read the committed JSON."""
 import base64
 import io
 import json
@@ -10,7 +10,7 @@ import os
 import sys
 import types
 
-REF = '/root/reference/python/bifrost'
+REF = os.path.join(os.environ.get('BIFROST_REFERENCE', '/root/reference'), 'python', 'bifrost')
 HERE = os.path.dirname(os.path.abspath(__file__))
 
 

@@ -15,7 +15,9 @@ from bifrost_b200.fdmt import Fdmt
 from oracle import fdmt as ofdmt
 
 sys.path.insert(0, os.path.dirname(os.path.abspath(__file__)))
-from golden.make_fdmt_golden import CASES as GOLDEN_CASES, SENTINEL  # noqa: E402
+from golden import digest  # noqa: E402
+from golden import make_ref_golden as refgold  # noqa: E402
+from golden.make_fdmt_golden import CASES as GOLDEN_CASES, SENTINEL, make_input  # noqa: E402
 
 GOLDEN = os.path.join(os.path.dirname(os.path.abspath(__file__)), 'golden', 'fdmt_ref_golden.npz')
 
@@ -36,12 +38,12 @@ def assert_same_bits(a, b):
 def test_oracle_matches_reference_golden(case):
     """Pins oracle/fdmt.py against outputs of the reference CUDA library."""
     name, ntime, nchan, md, f0, df, dtype, batch = case
-    g = np.load(GOLDEN)
-    x = g[name + '/in']
+    i = [c[0] for c in GOLDEN_CASES].index(name)
+    x = make_input(name, batch + (nchan, ntime), dtype, 1234 + i)
     x = x.astype(np.float32) if dtype == 'f32' else x
     out = np.full(batch + (md, ntime), SENTINEL, np.float32)
     ofdmt.fdmt(x, md, f0, df, out=out)
-    assert_same_bits(out, g[name + '/out'])
+    digest.check(np.load(GOLDEN), name + '/out', out, assert_same_bits)
 
 
 def test_oracle_dispersed_pulse_peaks_at_its_dm():
@@ -81,7 +83,6 @@ def run_gpu(x, md, f0, df, batch=(), negative_delays=False, sentinel=SENTINEL, w
 @pytest.mark.gpu
 @pytest.mark.parametrize("case", GOLDEN_CASES, ids=[c[0] for c in GOLDEN_CASES])
 def test_gpu_matches_oracle_bit_exact(case):
-    from golden.make_fdmt_golden import make_input
     name, ntime, nchan, md, f0, df, dtype, batch = case
     i = [c[0] for c in GOLDEN_CASES].index(name)
     x = make_input(name, batch + (nchan, ntime), dtype, 1234 + i)
@@ -91,7 +92,7 @@ def test_gpu_matches_oracle_bit_exact(case):
     ofdmt.fdmt(x, md, f0, df, out=want)
     assert_same_bits(got, want)
     if os.path.exists(GOLDEN):
-        assert_same_bits(got, np.load(GOLDEN)[name + '/out'])
+        digest.check(np.load(GOLDEN), name + '/out', got, assert_same_bits)
 
 
 @pytest.mark.gpu
@@ -190,32 +191,12 @@ def test_negative_delays_match_oracle():
 
 @pytest.mark.gpu
 def test_gpu_matches_reference_library():
-    """Same call sequence through both C ABIs on the same device buffers."""
-    import reflib
-    ref = reflib.load()
-    if ref is None:
-        pytest.skip("oracle/_ref/libbifrost_ref.so not present")
-    from bifrost_b200.libbifrost import _check
-    rng = np.random.default_rng(7)
-    for (ntime, nchan, md, dtype) in [(2000, 256, 301, np.float32), (1500, 100, 64, np.int8),
-                                     (4096, 512, 130, np.int8), (333, 17, 40, np.uint16)]:
-        if dtype == np.float32:
-            x = rng.normal(size=(nchan, ntime)).astype(np.float32)
-        else:
-            info = np.iinfo(dtype)
-            x = rng.integers(max(info.min, -127), min(info.max, 127) + 1, size=(nchan, ntime)).astype(dtype)
-        f0, df = 1000., 400. / nchan
-        got = run_gpu(x, md, f0, df)
-        d_in = bf.asarray(x, space='cuda')
-        d_out = bf.asarray(np.full((md, ntime), SENTINEL, np.float32), space='cuda')
-        plan = ctypes.c_void_p()
-        _check(ref.bfFdmtCreate(ctypes.byref(plan)))
-        _check(ref.bfFdmtInit(plan, nchan, md, f0, df, -2.0, 2, None, None))
-        _check(ref.bfFdmtExecute(plan, d_in.as_BFarray(), d_out.as_BFarray(), 0, None, None))
-        _check(ref.bfStreamSynchronize())
-        want = np.asarray(d_out.copy('system'))
-        _check(ref.bfFdmtDestroy(plan))
-        assert_same_bits(got, want)
+    """Bit for bit what the reference's own bfFdmtExecute computed for the same
+    inputs (tests/golden/ref_golden.npz, tests/golden/make_ref_golden.py)."""
+    g = np.load(refgold.GOLDEN)
+    for ntime, nchan, md, x in refgold.fdmt_inputs():
+        got = run_gpu(x, md, 1000., 400. / nchan)
+        digest.check(g, refgold.fdmt_key(ntime, nchan, md, x), got, assert_same_bits)
 
 
 @pytest.mark.gpu

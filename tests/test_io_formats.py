@@ -93,7 +93,9 @@ def fil_header(nchan, npol, dtype):
     return {'_tensor': {'dtype': dtype, 'shape': [-1, npol, nchan], 'labels': ['time', 'pol', 'freq'],
                         'scales': [[1500000000.0, 1e-3], None, [1500.0, -0.5]], 'units': ['s', None, 'MHz']},
             'name': 'obs', 'gulp_nframe': 16, 'source_name': 'FAKE', 'telescope': 'GBT', 'machine': 'GUPPI',
-            'coord_frame': 'topocentric', 'refdm': 0.0, 'refdm_units': 'pc cm^-3'}
+            'coord_frame': 'topocentric', 'refdm': 0.0, 'refdm_units': 'pc cm^-3',
+            # a source block's full path, longer than a sigproc header string holds
+            'rawdatafile': '/data/' + 'd' * 100 + '/obs.raw'}
 
 
 @pytest.mark.parametrize("dtype,npdt", [('f32', np.float32), ('i8', np.int8), ('u8', np.uint8)])
@@ -112,6 +114,7 @@ def test_sigproc_filterbank_round_trip(tmp_path, dtype, npdt):
     assert h['tstart'] == pytest.approx(1500000000.0 / 86400. + 40587) and h['tsamp'] == 1e-3
     assert (h['fch1'], h['foff']) == (1500.0, -0.5) and h['telescope_id'] == 6 and h['machine_id'] == 20
     assert h.get('signed', 0) == (1 if dtype == 'i8' else 0)
+    assert h['rawdatafile'] == 'obs.raw'
     np.testing.assert_array_equal(body.reshape(x.shape), x)
     out = Collect()
     with Pipeline() as p:
@@ -122,6 +125,13 @@ def test_sigproc_filterbank_round_trip(tmp_path, dtype, npdt):
     assert t['dtype'] == dtype and t['shape'] == [-1, 2, 32] and t['labels'] == ['time', 'pol', 'freq']
     assert out.headers[0]['telescope'] == 'GBT'
     np.testing.assert_array_equal(np.concatenate(out.chunks, 0), x)
+
+
+def test_sigproc_header_string_a_reader_cannot_take_is_an_error():
+    """Strings of 80 bytes or more would make a file no sigproc reader parses."""
+    sigproc.write_header(dict(source_name='x' * 79), io.BytesIO())
+    with pytest.raises(ValueError):
+        sigproc.write_header(dict(source_name='x' * 80), io.BytesIO())
 
 
 def test_sigproc_file_without_id_cards_round_trips(tmp_path):

@@ -126,33 +126,26 @@ def test_errors():
 
 
 def test_reduce_matches_the_reference_library():
-    """Same BFarray structs through the reference's own bfReduce (oracle/_ref,
-    src/reduce.cu:881-920) and ours: bit-identical for sum / min / max on float
-    data (same left-to-right order), 1 ulp for mean / stderr."""
+    """What the reference's own bfReduce (src/reduce.cu:881-920) computed for the
+    same inputs (tests/golden/ref_golden.npz, tests/golden/make_ref_golden.py):
+    bit-identical for sum / min / max on float data (same left-to-right order),
+    1 ulp for mean."""
     import os
     import sys
     sys.path.insert(0, os.path.dirname(os.path.abspath(__file__)))
-    import reflib
-    ref = reflib.load()
-    if ref is None or not hasattr(ref, 'bfReduce'):
-        pytest.skip("oracle/_ref/libbifrost_ref.so not present")
-    from bifrost_b200.libbifrost import _bf, _check
-    rng = np.random.default_rng(11)
-    ops = dict(sum=_bf.BF_REDUCE_SUM, min=_bf.BF_REDUCE_MIN, max=_bf.BF_REDUCE_MAX, mean=_bf.BF_REDUCE_MEAN,
-               pwrsum=_bf.BF_REDUCE_POWER_SUM)
-    for shape, axis, n in [((4096, 256), 1, 4), ((4096, 256), 0, 8), ((4, 65536), 1, 4), ((20, 40, 60), 1, 5)]:
-        a = rng.normal(size=shape).astype(np.float32)
+    from golden import digest
+    from golden import make_ref_golden as refgold
+    g = np.load(refgold.GOLDEN)
+    for shape, axis, n, a in refgold.reduce_inputs():
         oshape = list(shape)
         oshape[axis] //= n
         d_a = bf.asarray(a, space='cuda')
-        for name, code in ops.items():
+        for name in refgold.REDUCE_OPS:
             d_o = bf.empty(oshape, 'f32', 'cuda')
-            d_r = bf.empty(oshape, 'f32', 'cuda')
             bf.reduce(d_a, d_o, name)
-            _check(ref.bfReduce(d_a.as_BFarray(), d_r.as_BFarray(), code))
-            _check(ref.bfStreamSynchronize())
-            ours, theirs = np.asarray(d_o.copy('system')), np.asarray(d_r.copy('system'))
-            if name in ('sum', 'min', 'max', 'pwrsum'):
-                np.testing.assert_array_equal(ours, theirs, err_msg=str((shape, axis, n, name)))
+            ours = np.asarray(d_o.copy('system'))
+            key = refgold.reduce_key(shape, axis, n, name)
+            if name in refgold.REDUCE_EXACT:
+                digest.check(g, key, ours, lambda o, t: np.testing.assert_array_equal(o, t, err_msg=key))
             else:
-                np.testing.assert_allclose(ours, theirs, rtol=2e-7, err_msg=str((shape, axis, n, name)))
+                digest.check_close(g, key, ours, rtol=2e-7)

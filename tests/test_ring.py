@@ -1,13 +1,12 @@
 """bfRing* / bfProcLog* / bfAffinity* of libbifrost_b200.so (csrc/ring.cpp)
 against the reference's own ring.
 
-Parity is pinned two ways:
-  * tests/golden/ring_traces.json.gz -- scripts of calls with the answers the
-    reference's unmodified src/ring_impl.cpp gave (tests/golden/make_ring_golden.py);
-    replayed here call by call, no reference needed;
-  * live, when oracle/_ref/libbifrost_ref_ring.so is present (built by
-    oracle/ref_ring_build.sh; it travels to the GPU box): fresh random scripts
-    on both libraries.
+Parity is pinned by tests/golden/ring_traces.json.gz: random scripts of calls
+with the answers the reference's unmodified src/ring_impl.cpp gave
+(tests/golden/make_ring_golden.py), replayed here call by call, no reference
+needed.  When oracle/_ref/libbifrost_ref_ring.so is present (built by
+oracle/ref_ring_build.sh), the stored answers and the threaded expectations
+below are also checked against the reference's ring itself.
 The remaining tests exercise what a single-threaded script cannot: blocking
 calls between threads, and rings in device memory (-m gpu).
 """
@@ -29,9 +28,9 @@ REF = rt.load_reference()
 needs_ref = pytest.mark.skipif(REF is None, reason='oracle/_ref/libbifrost_ref_ring.so not built')
 
 
-def golden_cases():
+def golden_cases(key='cases'):
     with gzip.open(os.path.join(HERE, 'golden', 'ring_traces.json.gz')) as f:
-        return json.loads(f.read().decode())['cases']
+        return json.loads(f.read().decode())[key]
 
 
 def assert_same_trace(script, want, got):
@@ -54,11 +53,13 @@ def test_golden_traces_are_what_the_reference_does():
     assert rt.replay(REF, case['script']) == case['trace']
 
 
-@needs_ref
 @pytest.mark.timeout(300)
 @pytest.mark.parametrize('seed', range(100, 112))
 def test_live_differential_against_the_reference_ring(seed):
-    script, want = rt.generate(REF, seed, 350)
+    """Longer random scripts, built adaptively against the reference's ring
+    (ringtrace.generate) and stored with its answers."""
+    case, = [c for c in golden_cases('differential') if c['seed'] == seed]
+    script, want = case['script'], case['trace']
     assert len(script) > 100
     assert_same_trace(script, want, rt.replay(OURS, script))
 
